@@ -18,6 +18,8 @@ batch-1 greedy decode after a short prompt.  One "step" = one decoded token (for
           launch per token, CUDA events over the timed region); for the per-op graph path the GEMV launches' summed
           durations come from device-side %globaltimer stamps inside one replayed graph (tools/ktrace.py child process).
           step_frac = the same bytes / whole-step time (the north-star "fraction of HBM roofline"); peak = MEASURED_PEAKS.json.
+  --dump-outputs DIR : after the timed steps, DIR/tokens.npy holds the token id each timed step returned, as float64.  Weights
+          and prompt are seeded, so two builds run with the same arguments can be compared token for token.
   cpu_baseline : the oracle driving the reference's own C kernels (oracle/_ref) on a bounded sample, with Jlama's default
           thread count (half the available CPUs); `--impl reference` uses all of them.
   config.prefill : tokens/s of a 2048-token prompt on the tcgen05 prefill path (N = 1 only).
@@ -216,6 +218,12 @@ def config3_workload(ctx, cfg, peak, sessions=8, prompt_tokens=2048, decode_toke
     return out
 
 
+def dump_tokens(directory, tokens):
+    """--dump-outputs: the token ids the timed steps returned (float64 holds them exactly)."""
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "tokens.npy"), np.asarray(tokens, dtype=np.float64))
+
+
 def teacher_forced_logits(model, prompt, ref_tokens):
     """Feed the GPU the REFERENCE's tokens (every rank of a tensor-parallel job runs this with the same tokens): logits per step."""
     n = len(ref_tokens)
@@ -308,11 +316,15 @@ def run_reference_arm(args):
         tok, _ = m.sample(hidden)
         pos += 1
     t0 = time.time()
+    toks = []
     for _ in range(args.steps):
         hidden = m.batch_forward([tok], pos)
         tok, _ = m.sample(hidden)
+        toks.append(tok)
         pos += 1
     dt = time.time() - t0
+    if args.dump_outputs:
+        dump_tokens(args.dump_outputs, toks)
     val = args.steps / dt
     cores = o.num_threads()
     out = {
@@ -346,7 +358,10 @@ def main():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-config3", action="store_true", help="skip the BASELINE config-3 measurement (8B Q8_0, 8 sessions, prefill 2048 / decode 128)")
     ap.add_argument("--no-persistent", action="store_true", help="decode through the CUDA graph of per-op kernels instead of the persistent kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the token ids of the timed steps to DIR/tokens.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     capture_stdout()
 
@@ -618,6 +633,8 @@ def main():
         except Exception as e:  # noqa: BLE001 -- diagnostics must never break the bench line
             log("[bench] in-graph timeline skipped: %r" % (e,))
     if rank == 0:
+        if args.dump_outputs:
+            dump_tokens(args.dump_outputs, toks)
         emit(result)
     if dist is not None:
         dist.barrier()

@@ -1,8 +1,9 @@
-"""CPU tests: the oracle against the reference's golden vectors and the reference's own C kernels.
+"""CPU tests: the oracle against the reference's golden vectors and stored outputs of the reference's own C kernels.
 
 These pin the oracle (task rule: an oracle must be checked against every golden vector / fixture the
 reference's tests hold for the path, or against outputs of the reference itself).
 """
+import hashlib
 import json
 import os
 
@@ -34,56 +35,99 @@ def test_float_types_roundtrip(oracle):
     assert b[3] == 0x7FC0 and b[4] == 0x7F80 and b[5] == 0xFF80 and b[6] == 0
 
 
-@pytest.fixture(scope="module")
-def ref_kernels(oracle):
-    label = oracle.load_reference_kernels()
-    if label is None:
-        pytest.skip("oracle/_ref not built (no reference tree and no prebuilt kernels)")
-    yield label
-    oracle.use_reference_kernels(False)
+# Outputs of the reference's own C kernels (jlama-native/src/main/c/simd/vector_simd.c) on the seeded inputs built below, stored by
+# tests/golden/make_golden.py: "matches the reference" is checked on every machine, whether or not the reference's sources are at hand.
+# The kernels ship a 512-bit and a 256-bit body of every kernel (vector_simd.c:465-468); "avx512" is the AVX-512 VNNI build, "avx2" the
+# x86-64-v3 one.
+REF_GOLDEN = os.path.join(HERE, "golden", "ref_kernels.npz")
+GEMM_SHAPES = [(1, 128, 1024), (8, 64, 256), (32, 128, 1024), (7, 33, 512), (3, 16, 256)]
+GEMM_8B_SHAPES = [(1, 320, 4096), (8, 320, 4096), (1, 320, 14336), (8, 160, 14336)]
 
 
-@pytest.mark.parametrize("M,N,K", [(1, 128, 1024), (8, 64, 256), (32, 128, 1024), (7, 33, 512), (3, 16, 256)])
-def test_gemm_restatement_matches_reference_c_kernels(oracle, ref_kernels, M, N, K):
+def digest(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def gemm_inputs(M, N, K):
     # the reference's own distributions (TestOperations.java:94-109): A ~ U(-1,100), W ~ U(0,1)
     rng = np.random.default_rng(M * 1000 + N)
-    a = rng.uniform(-1, 100, (M, K)).astype(np.float32)
-    w = rng.uniform(0, 1, (N, K)).astype(np.float32)
+    return rng.uniform(-1, 100, (M, K)).astype(np.float32), rng.uniform(0, 1, (N, K)).astype(np.float32)
+
+
+def gemm_8b_inputs(M, N, K):
+    rng = np.random.default_rng(K + M)
+    return rng.standard_normal((M, K)).astype(np.float32), (rng.standard_normal((N, K)) * 0.02).astype(np.float32)
+
+
+def builds_inputs():
+    rng = np.random.default_rng(77)
+    return rng.standard_normal((4, 4096)).astype(np.float32), (rng.standard_normal((320, 4096)) * 0.02).astype(np.float32)
+
+
+def dense_inputs():
+    rng = np.random.default_rng(5)
+    return rng.uniform(-1, 100, (5, 512)).astype(np.float32), rng.uniform(0, 1, (20, 512)).astype(np.float32)
+
+
+def bf16_inputs():
+    rng = np.random.default_rng(9)
+    return rng.uniform(-1, 100, (4, 256)).astype(np.float32), rng.uniform(0, 1, (20, 256)).astype(np.float32)
+
+
+def q4_products(oracle, a, w):
+    """Q8 x Q4 and F32 x Q4 batch_dot of a and w through the reference's quantisers: the restatement, or the reference's kernels
+    after oracle.use_reference_kernels(True)."""
+    K, N = a.shape[1], w.shape[0]
     bq, bs = oracle.quantize_q4(w)
     aq, as_ = oracle.quantize_q8_act(a)
-    A8, Af, B = oracle.OTensor(oracle.I8, aq, as_), oracle.f32(a), oracle.OTensor(oracle.Q4, bq, bs)
-    oracle.use_reference_kernels(False)
-    r_q8, r_f32 = oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(Af, B, 0, 0, K, 0, 0, N)
-    oracle.use_reference_kernels(True)
-    q_q8, q_f32 = oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(Af, B, 0, 0, K, 0, 0, N)
-    oracle.use_reference_kernels(False)
+    B = oracle.OTensor(oracle.Q4, bq, bs)
+    return oracle.batch_dot(oracle.OTensor(oracle.I8, aq, as_), B, 0, 0, K, 0, 0, N), oracle.batch_dot(oracle.f32(a), B, 0, 0, K, 0, 0, N)
+
+
+@pytest.fixture(scope="module")
+def ref_out():
+    with np.load(REF_GOLDEN) as z:
+        return {k: z[k] for k in z.files}
+
+
+def reference(ref_out, key, *inputs):
+    """The stored outputs of case `key`, after checking that this machine built the inputs they were computed on."""
+    assert str(ref_out[key + ".inputs_sha256"]) == digest(*inputs), "%s: seeded inputs differ from those of %s" % (key, REF_GOLDEN)
+    return lambda name: ref_out[key + "." + name]
+
+
+@pytest.mark.parametrize("M,N,K", GEMM_SHAPES)
+def test_gemm_restatement_matches_reference_c_kernels(oracle, ref_out, M, N, K):
+    a, w = gemm_inputs(M, N, K)
+    ref = reference(ref_out, "gemm_%dx%dx%d" % (M, N, K), a, w)
+    r_q8, r_f32 = q4_products(oracle, a, w)
+    q_q8, q_f32 = ref("q8.avx512"), ref("f32.avx512")
     assert np.abs(r_q8 - q_q8).max() <= 2e-6 * np.abs(q_q8).max()
     assert np.abs(r_f32 - q_f32).max() <= 5e-6 * np.abs(q_f32).max()
     # and against the Naive control (get()*get() sequential), the reference tests' 1 % bar on the sum
-    naive = oracle.batch_dot(Af, B, 0, 0, K, 0, 0, N, naive=True)
+    B = oracle.OTensor(oracle.Q4, *oracle.quantize_q4(w))
+    naive = oracle.batch_dot(oracle.f32(a), B, 0, 0, K, 0, 0, N, naive=True)
     assert abs(naive.sum() - r_f32.sum()) <= 0.01 * abs(naive.sum())
     assert abs(naive.sum() - r_q8.sum()) <= 0.01 * abs(naive.sum())
 
 
-@pytest.mark.parametrize("M,N,K", [(1, 320, 4096), (8, 320, 4096), (1, 320, 14336), (8, 160, 14336)])
-def test_gemm_restatement_matches_reference_c_kernels_at_the_8b_reduction_lengths(oracle, ref_kernels, M, N, K):
+@pytest.mark.parametrize("M,N,K", GEMM_8B_SHAPES)
+def test_gemm_restatement_matches_reference_c_kernels_at_the_8b_reduction_lengths(oracle, ref_out, M, N, K):
     """The same pinning in the regime the benchmark runs in: K = 4096 (q/k/v/o, gate/up) and K = 14336 (down_proj) of Llama-3-8B, weights
     N(0, 0.02^2) through the reference's Q4 quantiser, activations N(0, 1) through its Q8 quantiser.  The two differ by summation order
     only; the float64 product of the dequantised operands bounds both."""
-    rng = np.random.default_rng(K + M)
-    a = rng.standard_normal((M, K)).astype(np.float32)
-    w = (rng.standard_normal((N, K)) * 0.02).astype(np.float32)
-    bq, bs = oracle.quantize_q4(w)
-    aq, as_ = oracle.quantize_q8_act(a)
-    A8, Af, B = oracle.OTensor(oracle.I8, aq, as_), oracle.f32(a), oracle.OTensor(oracle.Q4, bq, bs)
-    oracle.use_reference_kernels(False)
-    r_q8, r_f32 = oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(Af, B, 0, 0, K, 0, 0, N)
-    oracle.use_reference_kernels(True)
-    q_q8, q_f32 = oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(Af, B, 0, 0, K, 0, 0, N)
-    oracle.use_reference_kernels(False)
+    a, w = gemm_8b_inputs(M, N, K)
+    ref = reference(ref_out, "gemm8b_%dx%dx%d" % (M, N, K), a, w)
+    r_q8, r_f32 = q4_products(oracle, a, w)
+    q_q8, q_f32 = ref("q8.avx512"), ref("f32.avx512")
     assert not np.array_equal(r_f32, q_f32)  # two implementations really ran
     assert np.abs(r_q8 - q_q8).max() <= 3e-6 * np.abs(q_q8).max()
     assert np.abs(r_f32 - q_f32).max() <= 1e-5 * np.abs(q_f32).max()
+    bq, bs = oracle.quantize_q4(w)
+    aq, as_ = oracle.quantize_q8_act(a)
     wd = oracle.dequantize_q4(bq, bs).astype(np.float64)
     exact_f32 = a.astype(np.float64) @ wd.T
     exact_q8 = (aq.astype(np.float64).reshape(M, K // 32, 32) * as_.astype(np.float64)[:, :, None]).reshape(M, K) @ wd.T
@@ -91,61 +135,39 @@ def test_gemm_restatement_matches_reference_c_kernels_at_the_8b_reduction_length
         assert np.abs(got - exact).max() <= 1e-5 * np.abs(exact).max()
 
 
-def test_both_reference_builds_bracket_the_restatement(oracle, ref_kernels):
-    """The reference ships 256-bit and 512-bit bodies of every kernel (vector_simd.c:465-468); they sum in different orders, so they
-    differ from each other by as much as either differs from the restatement -- the yardstick for every "matches the reference" bar."""
-    labels = {}
-    for build in ("avx512", "avx2"):
-        lab = oracle.load_reference_kernels(build)
-        if lab is not None:
-            labels[build] = lab
-    if len(labels) < 2:
-        oracle.load_reference_kernels()
-        pytest.skip("this CPU runs only one of the reference's builds")
-    M, N, K = 4, 320, 4096
-    rng = np.random.default_rng(77)
-    a = rng.standard_normal((M, K)).astype(np.float32)
-    bq, bs = oracle.quantize_q4((rng.standard_normal((N, K)) * 0.02).astype(np.float32))
-    aq, as_ = oracle.quantize_q8_act(a)
-    A8, B = oracle.OTensor(oracle.I8, aq, as_), oracle.OTensor(oracle.Q4, bq, bs)
-    out = {}
-    for build in ("avx512", "avx2"):
-        oracle.load_reference_kernels(build)
-        oracle.use_reference_kernels(True)
-        out[build] = (oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(oracle.f32(a), B, 0, 0, K, 0, 0, N))
-    oracle.use_reference_kernels(False)
-    port = (oracle.batch_dot(A8, B, 0, 0, K, 0, 0, N), oracle.batch_dot(oracle.f32(a), B, 0, 0, K, 0, 0, N))
-    oracle.load_reference_kernels()  # back to the default build for the tests that follow
-    for i, bar in ((0, 3e-6), (1, 1e-5)):
+def test_both_reference_builds_bracket_the_restatement(oracle, ref_out):
+    """The reference's 256-bit and 512-bit bodies sum in different orders, so they differ from each other by as much as either
+    differs from the restatement -- the yardstick for every "matches the reference" bar."""
+    a, w = builds_inputs()
+    ref = reference(ref_out, "builds", a, w)
+    port = q4_products(oracle, a, w)
+    for i, kind, bar in ((0, "q8", 3e-6), (1, "f32", 1e-5)):
+        out = {b: ref(kind + "." + b) for b in ("avx512", "avx2")}
         scale = np.abs(port[i]).max()
-        d_builds = np.abs(out["avx512"][i] - out["avx2"][i]).max() / scale
-        d_port = max(np.abs(out[b][i] - port[i]).max() / scale for b in out)
+        d_builds = np.abs(out["avx512"] - out["avx2"]).max() / scale
+        d_port = max(np.abs(out[b] - port[i]).max() / scale for b in out)
         assert d_builds <= bar and d_port <= bar
         assert d_builds > 0  # the two builds are not bit-identical: bit-exactness against "the reference" is not defined for these sums
 
 
-def test_dense_f32_matches_reference_c_kernel(oracle, ref_kernels):
-    rng = np.random.default_rng(5)
-    a = rng.uniform(-1, 100, (5, 512)).astype(np.float32)
-    w = rng.uniform(0, 1, (20, 512)).astype(np.float32)
+def test_dense_f32_matches_reference_c_kernel(oracle, ref_out):
+    a, w = dense_inputs()
+    q = reference(ref_out, "dense_f32", a, w)("avx512")
     r = oracle.batch_dot(oracle.f32(a), oracle.f32(w), 0, 0, 512, 0, 0, 20)
-    q = oracle.ref_gemm_f32(a, w, 0, 20)
     assert np.abs(r - q).max() <= 5e-6 * np.abs(q).max()
 
 
-def test_f32_bf16_gemm_matches_reference_c_kernel(oracle, ref_kernels):
+def test_f32_bf16_gemm_matches_reference_c_kernel(oracle, ref_out):
     # F32 x BF16 (vector_simd.h:38; PanamaTensorOperations.java:1466-1539): N a multiple of 5 because of the reference
     # splitter's corner-tile bug (DESIGN.md section 6).  The reference's gemm_bf16 (BF16 x BF16, vector_simd.h:34) returns
     # NaNs / wrong sums for the same call shape when driven directly through its C entry point, so BF16 x BF16 is pinned
     # only against the exact float64 product below.
-    rng = np.random.default_rng(9)
-    a = rng.uniform(-1, 100, (4, 256)).astype(np.float32)
-    w = rng.uniform(0, 1, (20, 256)).astype(np.float32)
+    a, w = bf16_inputs()
+    q1 = reference(ref_out, "f32_bf16", a, w)("avx512")
     wb = oracle.f32_to_bf16(w)
     ab = oracle.f32_to_bf16(a)
     exact = oracle.bf16_to_f32(ab).astype(np.float64) @ oracle.bf16_to_f32(wb).astype(np.float64).T
     r1 = oracle.batch_dot(oracle.f32(a), oracle.OTensor(oracle.BF16, wb), 0, 0, 256, 0, 0, 20)
-    q1 = oracle.ref_gemm_f32_bf16(a, wb, 0, 20)
     assert np.abs(r1 - q1).max() <= 5e-6 * np.abs(q1).max()
     r2 = oracle.batch_dot(oracle.OTensor(oracle.BF16, ab), oracle.OTensor(oracle.BF16, wb), 0, 0, 256, 0, 0, 20)
     assert np.abs(r2 - exact).max() <= 5e-6 * np.abs(exact).max()
